@@ -27,6 +27,10 @@ all-gather, so total work is fixed (``"scaling": "strong"``).
 
 ``--impl reference`` times that CPU port alone (the reference's own implementation of the path
 is Whoosh, which is absent; see DESIGN.md) on the same config/metric/unit.
+
+``--dump-outputs DIR`` writes what the last timed step of ``value`` returned (``scores`` float32 [Q, k], 0 in the
+empty slots past ``counts``; ``docids``, ``counts`` and ``totals`` as float64) to ``DIR/<name>.npy``; the inputs
+depend only on the arguments, so two builds of the library can be compared output for output.
 """
 from __future__ import annotations
 
@@ -155,6 +159,39 @@ def measured_peak():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return FALLBACK_HBM_GBS, "fallback (B200_PROFILING.md)"
+
+
+#: --dump-outputs writes at most this many bytes; a larger batch is cut to a fixed, seeded sample of its queries
+DUMP_LIMIT_BYTES = 64_000_000 - 65_536       # (minus room for the .npy headers)
+
+
+def step_outputs(b):
+    """Host copies of what ``ShardedSearcher.run_plan`` hands its caller, per query: the top-k scores and docids in
+    W11 order, the length of that list and the match count.  Slots past the list's length (a query with fewer than k
+    matches) are decoded as score -inf and docid 0xFFFFFFFF; their score is written as 0 so that every value is
+    finite, and ``counts`` tells which slots hold hits."""
+    Q = b["totals"].numel()
+    k = b["scores"].numel() // Q
+    scores = b["scores"].cpu().numpy().reshape(Q, k)
+    counts = b["counts"].cpu().numpy().view(np.uint32)
+    live = np.arange(k)[None, :] < counts[:, None]
+    return {"scores": np.where(live, scores, 0).astype(np.float32),
+            "docids": b["docids"].cpu().numpy().view(np.uint32).reshape(Q, k).astype(np.float64),
+            "counts": counts.astype(np.float64),
+            "totals": b["totals"].cpu().numpy().view(np.uint64).astype(np.float64)}
+
+
+def write_outputs(path, arrays):
+    """``path/<name>.npy`` per array.  Above DUMP_LIMIT_BYTES only the rows of a seeded sample of the queries are
+    written, and their indices go to ``query_index.npy``."""
+    Q = arrays["totals"].shape[0]
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if Q * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(Q, DUMP_LIMIT_BYTES // (row_bytes + 8), replace=False))
+        arrays = dict({name: a[rows] for name, a in arrays.items()}, query_index=rows.astype(np.float64))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 #: DRAM traffic is not measured inside a bench run (it needs ncu's counters, and a number taken under a profiler is
@@ -307,7 +344,11 @@ def main():
                     help="engine option (a bm25f_options field, include/bm25f.h), e.g. --opt variant=3")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--check", type=int, default=200, help="queries checked against the oracle before timing")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results (scores, docids, counts, totals) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         log("note: the timing rules ask for >= 3 warm-up steps")
     if args.impl == "reference":
@@ -385,10 +426,12 @@ def main():
     barrier()
     ev0.record()
     for _ in range(args.steps):
-        ss.run_plan(plan)
+        last = ss.run_plan(plan)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    # the result buffers are reused by the e2e legs below, so the last step's results are copied out now
+    dumped = step_outputs(last) if args.dump_outputs and rank == 0 else None
     eng.synchronize()
     st = eng.stats()
     clk = clocks.stop() if rank == 0 else None
@@ -542,6 +585,8 @@ def main():
                "clocks": clk}
         if not args.no_cpu:
             out["cpu_baseline"] = cpu_baseline(ix, qs.queries, k)
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()
