@@ -330,18 +330,16 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 // Per tile of S documents the CTA owns, in shared memory:  acc[S] f32 score accumulators,
 // cnt[S] u8 "groups matched so far" counters and cand[S] u16 slots touched by the first
 // group.  Leaves are walked in group order (smallest group first) with a barrier between
-// leaves, so every accumulator is updated by one thread at a time, in a fixed order.
+// leaves, so every accumulator is updated by one thread at a time, in a fixed order: the plan's
+// leaf order, acc = fmaf(w, impact, acc) over the {docid, impact} pairs, as in the warp kernels,
+// so a document gets the same float32 score whichever kernel serves its query.
 // A posting of group g contributes only to slots with cnt == g (first hit of the group:
 // cnt becomes g + 1) or cnt == g + 1 (another leaf of the same group already hit).  After the
 // last leaf the candidates with cnt == n_groups are the tile's matches: they are counted,
 // turned into 64-bit keys and offered to the CTA's top-k buffer.
 // ------------------------------------------------------------------------------------------
 struct ScoreParams {
-  const uint32_t* docids;
-  const uint32_t* payload;
-  const uint8_t* lb;            // only when !packed
-  const uint8_t* deleted;       // or null
-  const float* norm;            // [n_fields * 256]
+  const uint2* pairs;           // {docid, impact} per posting (the warp kernels' store)
   const LeafRec* leaves;
   const QueryRec* queries;
   const ItemRec* items;
@@ -357,7 +355,6 @@ struct ScoreParams {
   unsigned long long* prof;     // BM25F_PROFILE builds: 16 cycle counters, else null
 };
 
-template <bool PACKED>
 __global__ void __launch_bounds__(512) k_score_topk(ScoreParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x;
@@ -416,20 +413,17 @@ __global__ void __launch_bounds__(512) k_score_topk(ScoreParams p) {
         const unsigned long long base = lf.off + lo;
         const unsigned long long end = lf.off + hi;
         const float w = lf.w;
-        const float* __restrict__ nrm = p.norm + lf.norm_off;
         const uint32_t g = lf.group;
-        // 16-byte aligned groups of four postings, one group per lane per step
+        // 32-byte aligned groups of four postings, one group per lane per step
         for (unsigned long long wb = (base & ~3ull) + (unsigned long long)warp * 128ull; wb < end;
              wb += (unsigned long long)nwarps * 128ull) {
           const unsigned long long i = wb + (unsigned long long)lane * 4ull;
-          uint32_t d[4] = {0, 0, 0, 0}, pl[4] = {0, 0, 0, 0};
-          uint32_t lbs = 0;
+          uint2 r[4] = {};
           if (i < end) {
-            const uint4 dv = __ldg(reinterpret_cast<const uint4*>(p.docids + i));
-            const uint4 pv = __ldg(reinterpret_cast<const uint4*>(p.payload + i));
-            d[0] = dv.x; d[1] = dv.y; d[2] = dv.z; d[3] = dv.w;
-            pl[0] = pv.x; pl[1] = pv.y; pl[2] = pv.z; pl[3] = pv.w;
-            if (!PACKED) lbs = __ldg(reinterpret_cast<const uint32_t*>(p.lb + i));
+            const uint4 a = __ldg(reinterpret_cast<const uint4*>(p.pairs + i));
+            const uint4 b = __ldg(reinterpret_cast<const uint4*>(p.pairs + i + 2));
+            r[0] = make_uint2(a.x, a.y); r[1] = make_uint2(a.z, a.w);
+            r[2] = make_uint2(b.x, b.y); r[3] = make_uint2(b.z, b.w);
           }
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
@@ -437,27 +431,22 @@ __global__ void __launch_bounds__(512) k_score_topk(ScoreParams p) {
             bool fresh = false;
             uint32_t slot = 0;
             if (valid) {
-              slot = d[e] - t0;
-              float tf;
-              uint32_t lb;
-              if (PACKED) { tf = (float)(pl[e] >> 8); lb = pl[e] & 255u; }
-              else { tf = __uint_as_float(pl[e]); lb = (lbs >> (8 * e)) & 255u; }
-              const float nv = __ldg(nrm + lb);
-              const float s = nv < 0.0f ? w * tf : __fdividef(w * tf, tf + nv);   // norm -1: field not scorable, the weight is the score (W15)
-              if (!(tf > 0.0f)) {
-                // tf == 0 marks a posting of a deleted document (W9): not a match
+              slot = r[e].x - t0;
+              const float u = __uint_as_float(r[e].y);
+              if (!(u > 0.0f)) {
+                // impact 0: a posting weight of 0 is not a match
               } else if (simple_or) {
                 const float old = acc[slot];
-                acc[slot] = old + s;
+                acc[slot] = fmaf(w, u, old);             // the warp kernels' arithmetic, in leaf order
                 fresh = (old == 0.0f);
               } else {
                 const uint32_t c = cnt[slot];
                 if (c == g) {
                   cnt[slot] = (uint8_t)(g + 1);
-                  acc[slot] += s;
+                  acc[slot] = fmaf(w, u, acc[slot]);
                   fresh = (g == 0);
                 } else if (c == g + 1) {
-                  acc[slot] += s;
+                  acc[slot] = fmaf(w, u, acc[slot]);
                 }
               }
             }
@@ -569,7 +558,7 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
 // The hot kernel, pipelined.  Same algorithm and data structures as k_score_topk, but DRAM
 // latency is decoupled from the per-leaf accumulate phases: the last warp of the CTA is a
 // PRODUCER that walks the item's static (tile, leaf, chunk) schedule ahead of the consumers and
-// stages posting chunks (docids + payload) into a ring of shared-memory stages with 1-D bulk
+// stages chunks of {docid, impact} pairs into a ring of shared-memory stages with 1-D bulk
 // copies (cp.async.bulk, completion on an mbarrier per stage).  The CONSUMER warps wait on the
 // stage's "full" barrier, accumulate one posting per lane from shared memory, release the stage
 // on its "empty" barrier, and synchronise among themselves (named barrier 1) only where the
@@ -598,16 +587,15 @@ struct __align__(16) StageMeta {   // 32 B: two 128-bit shared loads
   uint32_t vbeg;      // valid range inside the stage
   uint32_t vend;
   float w;            // leaf weight
-  uint32_t norm_off;  // field * 256
   uint32_t group;     // leaf's group rank
   uint32_t flags;
+  uint32_t pad;
 };
 
 struct PipeParams {
   ScoreParams sp;
   uint32_t chunk;       // postings per stage (multiple of 16)
   uint32_t stages;      // ring depth (<= PIPE_MAX_STAGES)
-  uint32_t nf_smem;     // fields whose norm table is copied to shared memory (0: read from global)
   uint32_t prune_at;    // sort + cut the key buffer when it holds this many keys
 };
 
@@ -619,7 +607,6 @@ struct PipeParams {
 // slots.  A document is offered to the top-k buffer only if its running score crosses the current
 // k-th best score ("hot"); until k hits exist the threshold is the smallest positive float, every
 // match is hot, the hot list overflows and the epilogue falls back to walking all candidates.
-template <bool PACKED>
 __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const ScoreParams& p = pp.sp;
@@ -635,11 +622,8 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
   float* acc = reinterpret_cast<float*>(keys + p.cap);
   uint16_t* cand = reinterpret_cast<uint16_t*>(acc + S);
   uint8_t* cnt = reinterpret_cast<uint8_t*>(cand + S);
-  uint32_t* sdoc = reinterpret_cast<uint32_t*>(smem_raw + (((size_t)p.cap * 8 + (size_t)S * 7 + 15) & ~(size_t)15));
-  uint32_t* spay = sdoc + (size_t)NS * CH;
-  uint8_t* slb = reinterpret_cast<uint8_t*>(spay + (size_t)NS * CH);
-  float* snorm = reinterpret_cast<float*>(slb + (PACKED ? 0 : (size_t)NS * CH));
-  uint16_t* hot = reinterpret_cast<uint16_t*>(snorm + (size_t)pp.nf_smem * 256);
+  uint2* spair = reinterpret_cast<uint2*>(smem_raw + (((size_t)p.cap * 8 + (size_t)S * 7 + 15) & ~(size_t)15));
+  uint16_t* hot = reinterpret_cast<uint16_t*>(spair + (size_t)NS * CH);
   __shared__ LeafRec s_leaf[MAXL];
   __shared__ uint32_t s_brow[PIPE_BROWS][MAXL];
   __shared__ StageMeta s_meta[PIPE_MAX_STAGES];
@@ -662,7 +646,6 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
 
   for (int i = tid; i < L; i += blockDim.x) s_leaf[i] = p.leaves[q.leaf_begin + i];
   for (uint32_t i = tid; i < S; i += blockDim.x) { acc[i] = 0.0f; cnt[i] = 0; }
-  for (uint32_t i = tid; i < pp.nf_smem * 256u; i += blockDim.x) snorm[i] = p.norm[i];
   if (tid == 0) {
     s_ncand[0] = 0; s_ncand[1] = 0; s_nhot[0] = 0; s_nhot[1] = 0; s_nkeys = 0; s_thr = 0ull; s_total = 0ull;
     s_thr_score = 1.17549435e-38f;    // FLT_MIN: every first hit crosses it
@@ -722,16 +705,14 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
               m.vbeg = (uint32_t)(a > c0 ? a - c0 : 0);
               m.vend = (uint32_t)(b < c0 + n ? b - c0 : n);
               m.w = lf.w;
-              m.norm_off = lf.norm_off;
               m.group = lf.group;
               const bool last_chunk = (c0 + CH >= b);
               m.flags = (last_chunk ? SF_LEAF_END : 0u) | ((last_chunk && l == last) ? SF_TILE_END : 0u) |
                         ((int)lf.group == G - 1 ? SF_LAST_GROUP : 0u);
+              m.pad = 0u;
               s_meta[stage] = m;
-              mbar_arrive_expect_tx(&s_full[stage], n * (PACKED ? 8u : 9u));
-              bulk_g2s(sdoc + (size_t)stage * CH, p.docids + c0, n * 4u, &s_full[stage]);
-              bulk_g2s(spay + (size_t)stage * CH, p.payload + c0, n * 4u, &s_full[stage]);
-              if (!PACKED) bulk_g2s(slb + (size_t)stage * CH, p.lb + c0, n, &s_full[stage]);
+              mbar_arrive_expect_tx(&s_full[stage], n * 8u);
+              bulk_g2s(spair + (size_t)stage * CH, p.pairs + c0, n * 8u, &s_full[stage]);
               if (++stage == NS) { stage = 0; phase ^= 1u; }
               PROF_ADD(3);                // [11] producer: meta + issue
             }
@@ -746,7 +727,7 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
     }
     if (lane == 0) {
       mbar_wait(&s_empty[stage], phase ^ 1u);
-      StageMeta m = {0u, 0u, 0u, 0u, 0.0f, 0u, 0u, SF_END};
+      StageMeta m = {0u, 0u, 0u, 0u, 0.0f, 0u, SF_END, 0u};
       s_meta[stage] = m;
       mbar_arrive(&s_full[stage]);
     }
@@ -770,10 +751,7 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
     {
       const float w = m.w;
       const float thr_s = s_thr_score;
-      const float* __restrict__ nrm = (pp.nf_smem ? snorm : p.norm) + m.norm_off;
-      const uint32_t* __restrict__ sd = sdoc + (size_t)stage * CH;
-      const uint32_t* __restrict__ spl = spay + (size_t)stage * CH;
-      const uint8_t* __restrict__ sl = slb + (size_t)stage * CH;
+      const uint2* __restrict__ sp = spair + (size_t)stage * CH;
       int* ncand_ctr = &s_ncand[seq & 1u];
       int* nhot_ctr = &s_nhot[seq & 1u];
       if (simple_or) {
@@ -782,17 +760,12 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
           bool fresh = false;
           uint32_t slot = 0;
           if (i >= m.vbeg && i < m.vend) {
-            const uint32_t pl = spl[i];
-            float tf;
-            uint32_t lb;
-            if (PACKED) { tf = (float)(pl >> 8); lb = pl & 255u; }
-            else { tf = __uint_as_float(pl); lb = sl[i]; }
-            if (tf > 0.0f) {                                    // tf == 0 marks a deleted document (W9)
-              slot = sd[i] - m.t0;
-              const float nv = nrm[lb];
-              const float s = nv < 0.0f ? w * tf : __fdividef(w * tf, tf + nv);   // norm -1: field not scorable (W15)
+            const uint2 r = sp[i];
+            const float u = __uint_as_float(r.y);
+            if (u > 0.0f) {                                     // impact 0: a posting weight of 0 is not a match
+              slot = r.x - m.t0;
               const float old = acc[slot];
-              const float nw = old + s;
+              const float nw = fmaf(w, u, old);                 // the warp kernels' arithmetic, in leaf order
               acc[slot] = nw;
               fresh = (old == 0.0f);
               if (nw >= thr_s && old < thr_s) {
@@ -818,19 +791,14 @@ __global__ void __launch_bounds__(544) k_score_pipe(PipeParams pp) {
           bool fresh = false, matched = false;
           uint32_t slot = 0;
           if (i >= m.vbeg && i < m.vend) {
-            slot = sd[i] - m.t0;
+            const uint2 r = sp[i];
+            slot = r.x - m.t0;
             const uint32_t c = cnt[slot];
             if (c == g || c == g + 1) {                         // alive: earlier groups all matched
-              const uint32_t pl = spl[i];
-              float tf;
-              uint32_t lb;
-              if (PACKED) { tf = (float)(pl >> 8); lb = pl & 255u; }
-              else { tf = __uint_as_float(pl); lb = sl[i]; }
-              if (tf > 0.0f) {
-                const float nv = nrm[lb];
-              const float s = nv < 0.0f ? w * tf : __fdividef(w * tf, tf + nv);   // norm -1: field not scorable (W15)
+              const float u = __uint_as_float(r.y);
+              if (u > 0.0f) {
                 const float old = acc[slot];
-                const float nw = old + s;
+                const float nw = fmaf(w, u, old);
                 acc[slot] = nw;
                 bool crossing = (nw >= thr_s);
                 if (c == g) {
@@ -1365,7 +1333,6 @@ struct bm25f_handle {
   // team kernel (variant 4): warps per CTA, target work per item, slices ahead to prefetch
   uint32_t tl_warps = 8, tl_slot_bytes = 10240, tl_split = 1u << 18, tl_prefetch = 0;
   uint32_t chunk = 512, stages = 4;   // pipeline geometry
-  uint32_t nf_smem = 0;
   int n_sms = 148;
   int ctas_per_sm = 0;
   int tl_ctas_per_sm = 0;
@@ -1460,8 +1427,7 @@ int key_capacity(int k, int nt) {
 
 size_t pipe_smem_bytes(const bm25f_handle* h, int cap) {
   size_t b = (score_smem_bytes(h->S, cap) + 15) & ~(size_t)15;
-  b += (size_t)h->stages * h->chunk * (h->packed ? 8 : 9);
-  b += (size_t)h->nf_smem * 256 * sizeof(float);
+  b += (size_t)h->stages * h->chunk * sizeof(uint2);
   b += (size_t)HOTCAP * sizeof(uint16_t);
   return b;
 }
@@ -1654,7 +1620,6 @@ int bm25f_create(const bm25f_index_desc* desc, int device, const bm25f_options* 
   }
   if (h->chunk < 64 || (h->chunk & 15) || h->chunk > 8192) { delete h; return fail(BM25F_EINVAL, "chunk_postings must be a multiple of 16 in 64..8192"); }
   if (h->stages < 2 || h->stages > (uint32_t)PIPE_MAX_STAGES) { delete h; return fail(BM25F_EINVAL, "stages must be 2..%d", PIPE_MAX_STAGES); }
-  h->nf_smem = desc->n_fields + 1 <= 4 ? desc->n_fields + 1 : 0;
   if (h->S < 256 || h->S > 65536 || (h->S & 3)) { delete h; return fail(BM25F_EINVAL, "tile_docs must be a multiple of 4 in 256..65536"); }
   if (h->NT < 64 || h->NT > 512 || (h->NT & 31)) { delete h; return fail(BM25F_EINVAL, "threads must be a multiple of 32 in 64..512"); }
   h->term_offsets.assign(desc->term_offsets, desc->term_offsets + desc->n_terms + 1);
@@ -1897,8 +1862,7 @@ int bm25f_create(const bm25f_index_desc* desc, int device, const bm25f_options* 
       CUH(cudaFuncGetAttributes(&fa, fn));
       CUH(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes));
     }
-    const void* fns[4] = {(const void*)k_score_topk<true>, (const void*)k_score_topk<false>,
-                          (const void*)k_score_pipe<true>, (const void*)k_score_pipe<false>};
+    const void* fns[2] = {(const void*)k_score_topk, (const void*)k_score_pipe};
     for (const void* fn : fns) {
       cudaFuncAttributes fa;
       CUH(cudaFuncGetAttributes(&fa, fn));
@@ -2755,11 +2719,7 @@ int bm25f_execute(bm25f_handle* h, bm25f_plan* p) {
   CU(cudaEventRecord(ev[1], st));
   if (p->n_items || p->n_w4 || p->n_w8 || p->n_is) {
     ScoreParams sp;
-    sp.docids = h->d_docids;
-    sp.payload = h->d_payload;
-    sp.lb = h->d_lb;
-    sp.deleted = nullptr;
-    sp.norm = h->d_norm;
+    sp.pairs = h->d_pairs;
     sp.leaves = p->d_leaves;
     sp.queries = p->d_queries;
     sp.items = p->d_items;
@@ -2888,13 +2848,10 @@ int bm25f_execute(bm25f_handle* h, bm25f_plan* p) {
       pp.sp = sp;
       pp.chunk = h->chunk;
       pp.stages = h->stages;
-      pp.nf_smem = h->nf_smem;
       pp.prune_at = (uint32_t)pipe_prune_at(p->k);
-      if (h->packed) k_score_pipe<true><<<p->n_items, h->NT + 32, p->smem_score, st>>>(pp);
-      else k_score_pipe<false><<<p->n_items, h->NT + 32, p->smem_score, st>>>(pp);
+      k_score_pipe<<<p->n_items, h->NT + 32, p->smem_score, st>>>(pp);
     } else {
-      if (h->packed) k_score_topk<true><<<p->n_items, h->NT, p->smem_score, st>>>(sp);
-      else k_score_topk<false><<<p->n_items, h->NT, p->smem_score, st>>>(sp);
+      k_score_topk<<<p->n_items, h->NT, p->smem_score, st>>>(sp);
     }
     if (p->n_items) {
       CU(cudaGetLastError());
@@ -2959,11 +2916,9 @@ int bm25f_execute(bm25f_handle* h, bm25f_plan* p) {
     } else if (p->n_w4) {
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_stream<1, false>, (int)h->st_warps * 32, stream_smem_bytes(h->st_warps, h->st_slot_bytes));
     } else if (!p->simple_kernel) {
-      if (h->packed) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_pipe<true>, (int)h->NT + 32, p->smem_score);
-      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_pipe<false>, (int)h->NT + 32, p->smem_score);
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_pipe, (int)h->NT + 32, p->smem_score);
     } else {
-      if (h->packed) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_topk<true>, (int)h->NT, p->smem_score);
-      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_topk<false>, (int)h->NT, p->smem_score);
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb_, k_score_topk, (int)h->NT, p->smem_score);
     }
     h->ctas_per_sm = nb_;
     h->stats.ctas_per_sm = (uint32_t)nb_;

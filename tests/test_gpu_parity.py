@@ -233,9 +233,14 @@ def test_sharded_equals_whole(cfg1):
         for i, r in enumerate(s.search_batch(qs.queries, limit=10)):
             tops[i].extend(r.top_n)
             totals[i] += len(r)
+    with Searcher(ix) as s:
+        whole = s.search_batch(qs.queries, limit=10)
     for i, q in enumerate(qs.queries):
         merged = sorted(tops[i], key=lambda t: (-t[0], t[1]))[:10]
         assert_query_parity(o, q, merged, totals[i], 10, ctx="query %d" % i)
+        if not qs.is_and[i] or qs.n_terms[i] == 1:
+            # one group: the same leaf order on every shard, the whole index's float32 scores bit for bit
+            assert merged == whole[i].top_n and totals[i] == len(whole[i]), "query %d" % i
 
 
 def test_every_field_and_cli_harness():
