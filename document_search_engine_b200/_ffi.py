@@ -29,6 +29,7 @@ EXPORTS = (
     "bm25f_set_stream", "bm25f_plan_destroy", "bm25f_search_batch", "bm25f_merge_keys", "bm25f_decode_keys", "bm25f_get_stats",
     "bm25f_reset_stats", "bm25f_submit", "bm25f_collect", "bm25f_set_final_date", "bm25f_fetch_final",
     "bm25f_plan_device_final", "bm25f_merge_final_lists", "bm25f_plan_gather_span", "bm25f_merge_gathered", "bm25f_put_lists",
+    "bm25f_put_positions", "bm25f_phrase_lists",
 )
 
 
@@ -106,6 +107,8 @@ def load_library(path: Optional[str] = None):
     lib.bm25f_synchronize.argtypes = [vp]
     lib.bm25f_set_stream.argtypes = [vp, vp, i32]
     lib.bm25f_put_lists.argtypes = [vp, u32, vp, vp, C.POINTER(u32)]
+    lib.bm25f_put_positions.argtypes = [vp, u32, vp, vp]
+    lib.bm25f_phrase_lists.argtypes = [vp, u32, vp, vp, vp, C.POINTER(u32)]
     lib.bm25f_plan_destroy.argtypes = [vp]
     lib.bm25f_plan_destroy.restype = None
     lib.bm25f_search_batch.argtypes = [vp, C.POINTER(QueryBatchDesc), i32, vp, vp, vp, vp]
@@ -286,6 +289,8 @@ class Engine:
         self.device = device
         self.n_fields = len(ix.field_names)
         self._weighting_key = None
+        #: fields whose word order is on the device (``put_positions``)
+        self.positions_fields = set()
 
     def set_weighting(self, norm: np.ndarray, key=None):
         norm = np.ascontiguousarray(norm, dtype=np.float32)
@@ -383,6 +388,32 @@ class Engine:
                 if lists else np.zeros(0, np.uint32))
         first = C.c_uint32()
         _check(self.lib, self.lib.bm25f_put_lists(self._h, len(lists), _ptr(offs), _ptr(docs), C.byref(first)))
+        return int(first.value)
+
+    def put_positions(self, field: int, offs: np.ndarray, ids: np.ndarray):
+        """Upload one field's word order (``FlatIndex.positions[field]``: document offsets, token ids in document order)
+        for the positional filter of ``phrase_lists``; replaces an earlier upload of the field."""
+        offs = np.ascontiguousarray(offs, dtype=np.int64)
+        if offs.shape != (self.n_docs_all + 1,):
+            raise ValueError("offsets must have n_docs_all + 1 = %d entries, got %r" % (self.n_docs_all + 1, offs.shape))
+        ids = np.ascontiguousarray(ids, dtype=np.int32)
+        if ids.size != int(offs[-1]) or int(offs[0]) != 0:
+            raise ValueError("the offsets must run from 0 to the number of tokens (%d)" % ids.size)
+        _check(self.lib, self.lib.bm25f_put_positions(self._h, int(field), _ptr(offs.view(np.uint64)), _ptr(ids.view(np.uint32))))
+        self.positions_fields.add(int(field))
+
+    def phrase_lists(self, words: Sequence[Sequence[int]], slops: Sequence[int]) -> int:
+        """The positional filter on the device (``bm25f_phrase_lists``): phrase ``i`` is the posting-list ids ``words[i]``
+        (``TERM_UNKNOWN`` for a word the index does not have) with ``slops[i]``.  Its live matching documents become
+        per-batch list ``i``, as ``put_lists`` makes them; returns the ``leaf_term`` id of the first one."""
+        wo = np.zeros(len(words) + 1, dtype=np.uint32)
+        if words:
+            np.cumsum([len(w) for w in words], out=wo[1:])
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(w, dtype=np.uint32) for w in words]) if words
+                                    else np.zeros(0, np.uint32))
+        sl = np.ascontiguousarray(slops, dtype=np.uint32)
+        first = C.c_uint32()
+        _check(self.lib, self.lib.bm25f_phrase_lists(self._h, len(words), _ptr(wo), _ptr(flat), _ptr(sl), C.byref(first)))
         return int(first.value)
 
     def stats(self) -> dict:

@@ -87,8 +87,9 @@ def doc_lengths(n_docs: int, seed: int, fieldno: int, spec: FieldSpec, device="c
 
 
 def _field_postings(n_docs: int, V: int, seed: int, fieldno: int, spec: FieldSpec, cdf: torch.Tensor,
-                    device, chunk_tokens: int):
-    """(sorted unique key=term*n_docs+doc, tf counts, lengths) for one field."""
+                    device, chunk_tokens: int, tokens: Optional[list] = None):
+    """(sorted unique key=term*n_docs+doc, tf counts, lengths) for one field.  ``tokens``: a list that receives the
+    field's ranks in document order (int32 chunks), when the caller wants the word order."""
     lengths = doc_lengths(n_docs, seed, fieldno, spec, device)
     csum = torch.cumsum(lengths, 0)
     keys_out, cnt_out = [], []
@@ -110,6 +111,8 @@ def _field_postings(n_docs: int, V: int, seed: int, fieldno: int, spec: FieldSpe
         del pos
         rank = torch.searchsorted(cdf, u, right=True).clamp_(max=V - 1)
         del u
+        if tokens is not None:
+            tokens.append(rank.to(torch.int32).cpu())
         key = rank * n_docs + doc
         del rank, doc
         key, _ = torch.sort(key)
@@ -126,15 +129,26 @@ def _field_postings(n_docs: int, V: int, seed: int, fieldno: int, spec: FieldSpe
 
 
 def make_corpus(n_docs: int, vocab: int, seed: int, fields: Sequence[FieldSpec] = (BODY,),
-                device: Optional[str] = None, chunk_tokens: int = 1 << 28, zipf_s: float = 1.0) -> FlatIndex:
-    """Generate the flattened index of a synthetic corpus."""
+                device: Optional[str] = None, chunk_tokens: int = 1 << 28, zipf_s: float = 1.0,
+                positions: bool = False) -> FlatIndex:
+    """Generate the flattened index of a synthetic corpus.  ``positions``: also keep every field's word order
+    (``FlatIndex.positions``: token ``fno * vocab + rank`` in document order), so that phrase queries can run on it."""
     if device is None:
         device = "cuda" if torch.cuda.is_available() else "cpu"
     cdf = torch.from_numpy(zipf_cdf(vocab, zipf_s)).to(device)
     offs_parts, doc_parts, tf_parts, lb_parts, totals = [], [], [], [], []
     base = 0
+    word_order = {}
     for fno, spec in enumerate(fields):
-        keys, cnts, lengths = _field_postings(n_docs, vocab, seed, fno, spec, cdf, device, chunk_tokens)
+        toks = [] if positions else None
+        keys, cnts, lengths = _field_postings(n_docs, vocab, seed, fno, spec, cdf, device, chunk_tokens, toks)
+        if positions:
+            po = np.zeros(n_docs + 1, dtype=np.int64)
+            np.cumsum(lengths.cpu().numpy(), out=po[1:])
+            ids = torch.cat(toks).numpy() if toks else np.zeros(0, np.int32)
+            ids += np.int32(fno * vocab)
+            word_order[fno] = (po, ids)
+            del toks
         term = torch.div(keys, n_docs, rounding_mode="floor")
         doc = keys - term * n_docs
         df = torch.bincount(term, minlength=vocab)
@@ -152,7 +166,7 @@ def make_corpus(n_docs: int, vocab: int, seed: int, fields: Sequence[FieldSpec] 
     return FlatIndex(field_names=[f.name for f in fields], n_docs_all=n_docs, term_offsets=term_offsets,
                      docids=np.concatenate(doc_parts), tfs=np.concatenate(tf_parts), term_field=term_field,
                      len_bytes=np.stack(lb_parts), field_length_total=np.array(totals, dtype=np.uint64),
-                     vocab_size=vocab)
+                     vocab_size=vocab, positions=word_order)
 
 
 # --------------------------------------------------------------------------

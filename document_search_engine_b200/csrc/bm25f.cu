@@ -13,6 +13,7 @@
 //   k_score_team      (team.cuh)          symmetric ANDs: CTA-built bounds table, private slices
 //   k_tile_bounds, k_score_pipe, k_score_topk   general fallback (k > 256, many leaves, paging, odd weights)
 //   k_merge_topk_warp / k_merge_topk      merge of per-item (or per-GPU) top-k lists
+//   k_phrase_mark / _scan / _compact (phrase.cuh)   phrase queries: positional filter -> per-batch document lists
 //   k_decode_keys                         keys -> (score, docid, count)
 #include "../../include/bm25f.h"
 
@@ -242,8 +243,10 @@ __global__ void k_compact_lists(const uint32_t* __restrict__ docids, const float
 // ------------------------------------------------------------------------------------------
 // Tile boundaries: bounds[q][j][l] = first posting of leaf l with docid >= j * S
 // ------------------------------------------------------------------------------------------
+// The docids are read from the {docid, impact} pairs: they line up with the compacted postings of the index and also
+// hold the per-batch lists (bm25f_put_lists / bm25f_phrase_lists) behind them.
 __global__ void k_tile_bounds(const LeafRec* __restrict__ leaves, uint32_t n_leaves, uint32_t T,
-                              uint32_t S, const uint32_t* __restrict__ docids,
+                              uint32_t S, const uint2* __restrict__ pairs,
                               uint32_t* __restrict__ bounds) {
   unsigned long long gid = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x;
   unsigned long long total = (unsigned long long)n_leaves * (T + 1);
@@ -256,10 +259,10 @@ __global__ void k_tile_bounds(const LeafRec* __restrict__ leaves, uint32_t n_lea
     lo = L.df;
   } else if (j > 0) {
     unsigned long long target = (unsigned long long)j * S;
-    const uint32_t* d = docids + L.off;
+    const uint2* d = pairs + L.off;
     while (lo < hi) {
       uint32_t mid = (lo + hi) >> 1;
-      if ((unsigned long long)__ldg(d + mid) < target) lo = mid + 1; else hi = mid;
+      if ((unsigned long long)__ldg(&d[mid].x) < target) lo = mid + 1; else hi = mid;
     }
   }
   size_t base = (size_t)L.qleaf0 * (T + 1);
@@ -983,6 +986,7 @@ __device__ __forceinline__ unsigned long long warp_topk_kth(const unsigned long 
 #include "team.cuh"
 #include "isect.cuh"
 #include "plan.cuh"
+#include "phrase.cuh"
 
 // ------------------------------------------------------------------------------------------
 // Merge of sorted top-k lists.  List l of query q starts at keys + start(q) + l * stride.
@@ -1343,6 +1347,15 @@ struct bm25f_handle {
   // n_terms + 1 + i (term n_terms is the padding between the two regions and is never valid)
   uint64_t dyn_base = 0, dyn_cap = 0;
   uint32_t dyn_terms = 0;
+  // word order of the fields (bm25f_put_positions), per field: token range of document d = [offs[d], offs[d + 1])
+  struct Positions {
+    unsigned long long* offs = nullptr;
+    uint32_t* toks = nullptr;
+    uint64_t bytes = 0;
+  };
+  std::vector<Positions> positions;
+  unsigned char* d_phrase = nullptr;    // grow-only workspace of bm25f_phrase_lists (records, flags, counts)
+  size_t d_phrase_cap = 0;
   bool compact_store = false;           // option: release the raw postings after the first bm25f_set_weighting
   bool raw_dropped = false;             // ... done: 8 bytes a posting stay; no re-weighting, no CTA-kernel queries
   std::vector<float> norm_host;         // the weighting in force (compact_store: the only one this handle will ever serve)
@@ -1514,6 +1527,11 @@ void bm25f_destroy(bm25f_handle* h) {
   cudaFree(h->d_prof);
   cudaFree(h->d_term_offsets);
   cudaFree(h->d_term_field);
+  for (auto& P : h->positions) {
+    cudaFree(P.offs);
+    cudaFree(P.toks);
+  }
+  cudaFree(h->d_phrase);
   if (h->h_ctr) cudaFreeHost(h->h_ctr);
   for (auto& A : h->arenas) {
     cudaFree(A.d);
@@ -1570,6 +1588,7 @@ int bm25f_create(const bm25f_index_desc* desc, int device, const bm25f_options* 
   h->n_postings = desc->n_postings;
   h->doc_base = desc->doc_base;
   h->n_fields = desc->n_fields;
+  h->positions.resize(h->n_fields);
   if (opts) {
     if (opts->tile_docs) h->S = opts->tile_docs;
     if (opts->threads) h->NT = opts->threads;
@@ -2331,7 +2350,7 @@ int prepare_impl(bm25f_handle* h, const bm25f_query_batch* b, int k, bm25f_plan*
     bool gseen[32];
     for (uint32_t g = 0; g < G; ++g) { gsize[g] = 0; gseen[g] = false; }
     uint32_t prev_g = 0, n_neg_in = 0;
-    bool all_pos = true, has_dyn = false;
+    bool all_pos = true;
     for (uint32_t i = a; i < e; ++i) {
       const uint32_t g = b->leaf_group[i];
       const bool neg = (g == BM25F_GROUP_NOT);             // a leaf of a NOT clause: excludes, never scores
@@ -2341,7 +2360,6 @@ int prepare_impl(bm25f_handle* h, const bm25f_query_batch* b, int k, bm25f_plan*
       const uint32_t term = resolve_term(h, b->leaf_term[i]);
       if (term != BM25F_TERM_UNKNOWN) {
         if (!valid_term(h, term)) PFAIL(BM25F_EINVAL, "query %u: leaf_term %u out of range", qi, b->leaf_term[i]);
-        if (term > h->n_terms) has_dyn = true;
         if (!neg) gsize[g] += h->term_offsets[term + 1] - h->term_offsets[term];
       }
       if (neg) { ++n_neg_in; continue; }
@@ -2429,9 +2447,6 @@ int prepare_impl(bm25f_handle* h, const bm25f_query_batch* b, int k, bm25f_plan*
                                    : g0 * (uint64_t)(nlq - 1) * h->is_ratio < P)));
     const bool use_team = !use_isect && stream_ok && qr.after_key == 0ull && n_neg == 0 && !final_mode && k <= 32 && (h->variant == 4 || (h->variant == 0 && !(qr.flags & QF_SIMPLE_OR)));
     const int cls = use_isect ? 3 : stream_ok ? (use_team ? 1 : 0) : 2;
-    if (cls == 2 && has_dyn)
-      PFAIL(BM25F_EINVAL, "query %u uses a bm25f_put_lists list and needs the CTA kernels (k > 256, more than 32 leaves, a non-positive "
-                          "weight or a paging bound): per-batch lists are served by the warp kernels only", qi);
     if (cls == 2 && h->raw_dropped)
       PFAIL(BM25F_EINVAL, "query %u needs the kernels that read the raw postings (k > 256, more than 32 leaves, a non-positive weight or a "
                           "paging bound) and the engine was created with compact_store", qi);
@@ -2712,7 +2727,7 @@ int bm25f_execute(bm25f_handle* h, bm25f_plan* p) {
   CU(cudaMemsetAsync(p->d_totals, 0, ((size_t)p->Q + 8) * 8, st));   // totals + the work counters
   const unsigned long long nb = p->n_items ? (unsigned long long)p->n_leaves * (p->T + 1) : 0ull;
   if (nb) {
-    k_tile_bounds<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(p->d_leaves, p->n_leaves, p->T, h->S, h->d_docids, p->d_bounds);
+    k_tile_bounds<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(p->d_leaves, p->n_leaves, p->T, h->S, h->d_pairs, p->d_bounds);
     CU(cudaGetLastError());
     ++launches;
   }
@@ -3155,30 +3170,25 @@ int bm25f_decode_keys(bm25f_handle* h, const uint64_t* d_keys, uint32_t n_querie
   return 0;
 }
 
-int bm25f_put_lists(bm25f_handle* h, uint32_t n_lists, const uint64_t* offsets, const uint32_t* docids, uint32_t* first_term) {
-  if (!h || !first_term || (n_lists && (!offsets || (offsets[n_lists] && !docids)))) return fail(BM25F_EINVAL, "null argument");
-  if (n_lists > BM25F_MAX_FILTER_LISTS) return fail(BM25F_EINVAL, "at most %d lists a batch", BM25F_MAX_FILTER_LISTS);
-  if (n_lists && offsets[0] != 0) return fail(BM25F_EINVAL, "offsets must start at 0");
-  const uint64_t total = n_lists ? offsets[n_lists] : 0;
-  if (total > h->dyn_cap) return fail(BM25F_EINVAL, "%llu postings in the lists, room for %llu (option filter_postings)", (unsigned long long)total, (unsigned long long)h->dyn_cap);
-  for (uint32_t l = 0; l < n_lists; ++l) {
-    if (offsets[l + 1] < offsets[l] || offsets[l + 1] > total) return fail(BM25F_EINVAL, "offsets not monotonic at list %u", l);
-    for (uint64_t i = offsets[l]; i < offsets[l + 1]; ++i)
-      if (docids[i] >= h->n_docs || (i > offsets[l] && docids[i] <= docids[i - 1]))
-        return fail(BM25F_EINVAL, "list %u: docids must be < n_docs_all and strictly ascending", l);
-  }
+}  // extern "C" (reopened below)
+
+namespace {
+
+constexpr size_t LIST_PAD = 1024;   // end markers behind the per-batch lists: rows and prefetches may read past the last posting
+
+// Per-batch lists: refused while a submitted batch is in flight; waits until nothing reads the previous lists.
+int begin_lists(bm25f_handle* h) {
   for (auto& A : h->arenas)
     if (A.submitted) return fail(BM25F_EINVAL, "a submitted batch is in flight: bm25f_collect it before replacing the lists");
   CU(cudaSetDevice(h->device));
   CU(cudaStreamSynchronize(h->stream));            // nothing may still be reading the previous lists
   CU(cudaStreamSynchronize(h->copy_stream));
-  // {docid, impact 1.0}, then a run of end markers: rows and prefetches may read past the last posting of the last list
-  const size_t pad = 1024;
-  std::vector<uint2> pairs(total + pad);
-  const uint32_t one = 0x3F800000u;
-  for (uint64_t i = 0; i < total; ++i) pairs[i] = make_uint2(docids[i], one);
-  for (size_t i = 0; i < pad; ++i) pairs[total + i] = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu);
-  CU(cudaMemcpyAsync(h->d_pairs + h->dyn_base, pairs.data(), pairs.size() * sizeof(uint2), cudaMemcpyHostToDevice, h->stream));
+  return 0;
+}
+
+// The lists are at dyn_base + offsets[l] .. dyn_base + offsets[l + 1] of `pairs` (written on the handle's stream, the
+// end markers included): make them leaf_term n_terms + 1 + l.
+int install_lists(bm25f_handle* h, uint32_t n_lists, const uint64_t* offsets, uint32_t* first_term) {
   // term table: [0, n_terms) the index, n_terms the padding between the regions, then the lists (pseudo-field n_fields)
   h->term_offsets.resize(h->n_terms + 1);
   h->term_field.resize(h->n_terms);
@@ -3194,6 +3204,152 @@ int bm25f_put_lists(bm25f_handle* h, uint32_t n_lists, const uint64_t* offsets, 
   CU(cudaStreamSynchronize(h->stream));            // (the sources are locals)
   *first_term = (uint32_t)h->n_terms + 1u;
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int bm25f_put_lists(bm25f_handle* h, uint32_t n_lists, const uint64_t* offsets, const uint32_t* docids, uint32_t* first_term) {
+  if (!h || !first_term || (n_lists && (!offsets || (offsets[n_lists] && !docids)))) return fail(BM25F_EINVAL, "null argument");
+  if (n_lists > BM25F_MAX_FILTER_LISTS) return fail(BM25F_EINVAL, "at most %d lists a batch", BM25F_MAX_FILTER_LISTS);
+  if (n_lists && offsets[0] != 0) return fail(BM25F_EINVAL, "offsets must start at 0");
+  const uint64_t total = n_lists ? offsets[n_lists] : 0;
+  if (total > h->dyn_cap) return fail(BM25F_EINVAL, "%llu postings in the lists, room for %llu (option filter_postings)", (unsigned long long)total, (unsigned long long)h->dyn_cap);
+  for (uint32_t l = 0; l < n_lists; ++l) {
+    if (offsets[l + 1] < offsets[l] || offsets[l + 1] > total) return fail(BM25F_EINVAL, "offsets not monotonic at list %u", l);
+    for (uint64_t i = offsets[l]; i < offsets[l + 1]; ++i)
+      if (docids[i] >= h->n_docs || (i > offsets[l] && docids[i] <= docids[i - 1]))
+        return fail(BM25F_EINVAL, "list %u: docids must be < n_docs_all and strictly ascending", l);
+  }
+  if (int rc = begin_lists(h)) return rc;
+  // {docid, impact 1.0}, then a run of end markers
+  std::vector<uint2> pairs(total + LIST_PAD);
+  const uint32_t one = 0x3F800000u;
+  for (uint64_t i = 0; i < total; ++i) pairs[i] = make_uint2(docids[i], one);
+  for (size_t i = 0; i < LIST_PAD; ++i) pairs[total + i] = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu);
+  CU(cudaMemcpyAsync(h->d_pairs + h->dyn_base, pairs.data(), pairs.size() * sizeof(uint2), cudaMemcpyHostToDevice, h->stream));
+  return install_lists(h, n_lists, offsets, first_term);
+}
+
+int bm25f_put_positions(bm25f_handle* h, uint32_t field, const uint64_t* doc_offsets, const uint32_t* tokens) {
+  if (!h || !doc_offsets) return fail(BM25F_EINVAL, "null argument");
+  if (field >= h->n_fields) return fail(BM25F_EINVAL, "field %u out of range (%u fields)", field, h->n_fields);
+  if (doc_offsets[0] != 0) return fail(BM25F_EINVAL, "doc_offsets must start at 0");
+  for (uint64_t d = 0; d < h->n_docs; ++d)
+    if (doc_offsets[d + 1] < doc_offsets[d]) return fail(BM25F_EINVAL, "doc_offsets not monotonic at document %llu", (unsigned long long)d);
+  const uint64_t n_tok = doc_offsets[h->n_docs];
+  if (n_tok && !tokens) return fail(BM25F_EINVAL, "null tokens");
+  CU(cudaSetDevice(h->device));
+  bm25f_handle::Positions P;
+  const size_t ob = (size_t)(h->n_docs + 1) * 8, tb = (size_t)n_tok * 4;
+  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&P.offs), ob);
+  if (e == cudaSuccess && tb) e = cudaMalloc(reinterpret_cast<void**>(&P.toks), tb);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(P.offs, doc_offsets, ob, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess && tb) e = cudaMemcpyAsync(P.toks, tokens, tb, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  if (e != cudaSuccess) {
+    cudaFree(P.offs);
+    cudaFree(P.toks);
+    return fail(e == cudaErrorMemoryAllocation ? BM25F_ENOMEM : BM25F_ECUDA, "uploading the word order of field %u: %s", field, cudaGetErrorString(e));
+  }
+  P.bytes = ob + tb;
+  bm25f_handle::Positions& old = h->positions[field];
+  cudaFree(old.offs);                              // (the stream was synchronised above: nothing reads them)
+  cudaFree(old.toks);
+  h->device_bytes = h->device_bytes - old.bytes + P.bytes;
+  h->stats.device_bytes = h->device_bytes;
+  old = P;
+  return 0;
+}
+
+int bm25f_phrase_lists(bm25f_handle* h, uint32_t n_phrases, const uint32_t* word_offsets, const uint32_t* words, const uint32_t* slops,
+                       uint32_t* first_term) {
+  if (!h || !first_term || (n_phrases && (!word_offsets || !slops || (word_offsets[n_phrases] && !words)))) return fail(BM25F_EINVAL, "null argument");
+  if (n_phrases > BM25F_MAX_FILTER_LISTS) return fail(BM25F_EINVAL, "at most %d lists a batch", BM25F_MAX_FILTER_LISTS);
+  if (n_phrases && word_offsets[0] != 0) return fail(BM25F_EINVAL, "word_offsets must start at 0");
+  // one record per phrase that has candidates: its rarest word's live postings
+  std::vector<PhraseRec> recs;
+  std::vector<uint32_t> rec_of(n_phrases, 0xFFFFFFFFu);
+  uint64_t n_flag_words = 0;
+  for (uint32_t i = 0; i < n_phrases; ++i) {
+    const uint32_t a = word_offsets[i], e = word_offsets[i + 1];
+    if (e < a) return fail(BM25F_EINVAL, "word_offsets not monotonic at phrase %u", i);
+    if (e - a > (uint32_t)PH_MAX_WORDS) return fail(BM25F_EINVAL, "phrase %u has %u words (at most %d)", i, e - a, PH_MAX_WORDS);
+    bool unknown = (e == a);
+    int field = -1;
+    uint32_t rare = 0;
+    uint64_t rare_df = ~0ull;
+    for (uint32_t j = a; j < e; ++j) {
+      const uint32_t t = words[j];
+      if (t == BM25F_TERM_UNKNOWN) { unknown = true; continue; }
+      if (t >= h->n_real_terms) return fail(BM25F_EINVAL, "phrase %u: word %u is not a posting list of the index", i, t);
+      const int f = h->term_field[t];
+      if (field >= 0 && f != field) return fail(BM25F_EINVAL, "phrase %u: its words belong to different fields", i);
+      field = f;
+      const uint64_t df = h->term_offsets[t + 1] - h->term_offsets[t];
+      if (df < rare_df) { rare_df = df; rare = t; }
+    }
+    if (field >= 0 && !h->positions[field].offs)
+      return fail(BM25F_EINVAL, "phrase %u: field %d has no word order on the device (bm25f_put_positions)", i, field);
+    if (unknown || rare_df == 0) continue;         // an unknown word or no live candidate: the empty list, no launch
+    PhraseRec r{};
+    r.offs = h->positions[field].offs;
+    r.toks = h->positions[field].toks;
+    r.cand = h->term_offsets[rare];
+    r.n_cand = (uint32_t)rare_df;
+    r.word0 = (uint32_t)n_flag_words;
+    r.n_words = e - a;
+    r.slop = slops[i];
+    for (uint32_t j = a; j < e; ++j) r.words[j - a] = words[j];
+    rec_of[i] = (uint32_t)recs.size();
+    recs.push_back(r);
+    n_flag_words += (rare_df + 31) / 32;
+    if (n_flag_words > 0x7FFFFFFFull) return fail(BM25F_EINVAL, "too many phrase candidates in one batch");
+  }
+  if (int rc = begin_lists(h)) return rc;
+  const uint32_t n_recs = (uint32_t)recs.size(), nfw = (uint32_t)n_flag_words;
+  const uint32_t n_chunks = (nfw + PH_CHUNK_WORDS - 1) / PH_CHUNK_WORDS;
+  const size_t o_recs = 0, o_flags = align_up((size_t)n_recs * sizeof(PhraseRec)), o_cnt = o_flags + align_up((size_t)nfw * 4),
+               o_chunk = o_cnt + align_up((size_t)n_recs * 4), need = o_chunk + align_up((size_t)n_chunks * 4);
+  std::vector<unsigned int> counts(n_recs, 0u);
+  if (n_recs) {
+    if (need > h->d_phrase_cap) {
+      cudaFree(h->d_phrase);                       // (begin_lists synchronised the stream)
+      h->d_phrase = nullptr;
+      h->d_phrase_cap = 0;
+      const size_t cap = align_up(need + need / 2, 1u << 20);
+      cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&h->d_phrase), cap);
+      if (e != cudaSuccess) return fail(BM25F_ENOMEM, "cudaMalloc(%zu): %s", cap, cudaGetErrorString(e));
+      h->d_phrase_cap = cap;
+    }
+    unsigned char* d = h->d_phrase;
+    const PhraseRec* d_recs = reinterpret_cast<const PhraseRec*>(d + o_recs);
+    uint32_t* d_flags = reinterpret_cast<uint32_t*>(d + o_flags);
+    unsigned int* d_cnt = reinterpret_cast<unsigned int*>(d + o_cnt);
+    unsigned int* d_chunk = reinterpret_cast<unsigned int*>(d + o_chunk);
+    CU(cudaMemcpyAsync(d + o_recs, recs.data(), (size_t)n_recs * sizeof(PhraseRec), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemsetAsync(d + o_cnt, 0, need - o_cnt, h->stream));
+    k_phrase_mark<<<nfw, 256, 0, h->stream>>>(d_recs, n_recs, h->d_pairs, d_flags, d_cnt, d_chunk);
+    CU(cudaGetLastError());
+    k_phrase_scan<<<1, 1024, 0, h->stream>>>(d_chunk, n_chunks);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(counts.data(), d_cnt, (size_t)n_recs * 4, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+  }
+  std::vector<uint64_t> offs(n_phrases + 1, 0);
+  for (uint32_t i = 0; i < n_phrases; ++i) offs[i + 1] = offs[i] + (rec_of[i] == 0xFFFFFFFFu ? 0u : counts[rec_of[i]]);
+  const uint64_t total = offs[n_phrases];
+  if (total > h->dyn_cap) return fail(BM25F_EINVAL, "%llu postings in the lists, room for %llu (option filter_postings)", (unsigned long long)total, (unsigned long long)h->dyn_cap);
+  if (total) {
+    unsigned char* d = h->d_phrase;
+    k_phrase_compact<<<n_chunks, 1024, 0, h->stream>>>(reinterpret_cast<const PhraseRec*>(d + o_recs), n_recs, h->d_pairs,
+                                                        reinterpret_cast<const uint32_t*>(d + o_flags), nfw,
+                                                        reinterpret_cast<const unsigned int*>(d + o_chunk), h->d_pairs + h->dyn_base);
+    CU(cudaGetLastError());
+  }
+  CU(cudaMemsetAsync(h->d_pairs + h->dyn_base + total, 0xFF, LIST_PAD * sizeof(uint2), h->stream));
+  return install_lists(h, n_phrases, offs.data(), first_term);
 }
 
 int bm25f_get_stats(bm25f_handle* h, bm25f_stats* out) {

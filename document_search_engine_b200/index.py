@@ -128,7 +128,8 @@ class FlatIndex:
             raise ValueError("scorable must have one entry per field")
         #: word order, for phrases (Whoosh: the ``positions`` posting format of a ``TEXT(phrase=True)`` field; reference
         #: ``my_index.py:172-177``): per field index ``f`` the documents' token sequences as posting-list ids,
-        #: ``(offsets[n_docs_all + 1], ids[sum of lengths])``, -1 for a token that is not indexed.  Host side only.
+        #: ``(offsets[n_docs_all + 1], ids[sum of lengths])``, -1 for a token that is not indexed.  A searcher uploads a
+        #: field's word order to the device the first time a phrase on the field reaches it (``bm25f_put_positions``).
         self.positions = {int(f): (np.ascontiguousarray(o, dtype=np.int64), np.ascontiguousarray(i, dtype=np.int32))
                           for f, (o, i) in (positions or {}).items()}
         self.schema = Schema(self.field_names, stored=self._stored_names())
@@ -375,7 +376,7 @@ class FlatIndex:
                          term_weight_total=self.term_weight_total, scorable=self.scorable,
                          positions={f: (o[lo:hi + 1] - o[lo], i[int(o[lo]):int(o[hi])]) for f, (o, i) in self.positions.items()})
 
-    # ---- phrases (host side; SURVEY.md section 8 f3) ----------------------------
+    # ---- phrases (CPU reference of the device filter, bm25f_phrase_lists; SURVEY.md section 8 f3) --------------
     def phrase_docs(self, fieldname, words: Sequence[object], slop: int = 1) -> np.ndarray:
         """Local docnums (ascending) in which ``words`` occur in this order, every word at most ``slop`` positions
         after the one before (``slop=1``: adjacent) - the documents Whoosh's ``Phrase(fieldname, words, slop)`` lets

@@ -354,10 +354,10 @@ class Phrase(Query):
     [W] ``Phrase.matcher``: a word that is not in the field -> NullMatcher; else the ``SpanNear`` chain of the words'
     term matchers, ordered, every word 1 .. ``slop`` positions after the one before (``slop=1``: adjacent), over an
     IntersectionMatcher - so a matching document scores the SUM of its words' BM25F scores, and the positions only
-    decide whether it matches.  The engine does the same in two steps: the host finds the documents that pass the
-    positional test (``FlatIndex.phrase_docs``, over the candidates of the rarest word), hands them to the library as a
-    per-batch posting list (``bm25f_put_lists``), and the query runs as ``And(words..., that list)`` - the list is
-    the smallest group, so the candidate-driven kernel walks it and looks the words' postings up."""
+    decide whether it matches.  The engine does the same in two steps: a positional filter on the device finds the
+    documents that pass (``bm25f_phrase_lists``, over the candidates of the rarest word; ``FlatIndex.phrase_docs`` is
+    its CPU reference) and keeps them as a per-batch posting list, and the query runs as ``And(words..., that list)`` -
+    the list is the smallest group, so the candidate-driven kernel walks it and looks the words' postings up."""
 
     def __init__(self, fieldname: str, words: Sequence[object], slop: int = 1, boost: float = 1.0):
         self.fieldname = fieldname

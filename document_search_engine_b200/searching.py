@@ -415,7 +415,7 @@ class Searcher:
         else:
             if has_phrase(q):
                 # a phrase is And(its words, the documents that pass the positional test): the latter is a per-batch
-                # list (bm25f_put_lists), numbered by ``register``; such a lowering is not remembered on the query
+                # list (bm25f_phrase_lists), numbered by ``register``; such a lowering is not remembered on the query
                 if register is None:
                     raise UnsupportedQuery("phrase queries are served by search() / search_page() / search_batch(), "
                                            "not by pre-packed batches: %r" % (q,))
@@ -490,9 +490,10 @@ class Searcher:
         terms = np.where(known, tids, _ffi.TERM_UNKNOWN).astype(np.uint32)
         if phrases:
             # [W] Phrase: the positions decide whether a document matches, the score is the words' alone.  The
-            # documents that pass go to the library as posting lists; their leaves get a weight far below float32
-            # resolution of any score (and above the library's "positive weight" bar)
-            first = self.engine.put_lists([self.ix.phrase_docs(p.fieldname, p.words, p.slop) for p in phrases])
+            # documents that pass (the positional filter runs on the device) become per-batch posting lists; their
+            # leaves get a weight far below float32 resolution of any score (and above the library's "positive
+            # weight" bar)
+            first = self._phrase_lists(phrases)
             flt = tids <= _FILTER_TID
             terms[flt] = (first + (_FILTER_TID - tids[flt])).astype(np.uint32)
             w[flt] = FILTER_WEIGHT
@@ -501,6 +502,25 @@ class Searcher:
             terms[ev] = (_ffi.TERM_EVERY_BASE + (-2 - tids[ev])).astype(np.uint32)
             w[ev] = rec["boost"][ev]
         return _ffi.PackedBatch(offs, np.asarray(ngroups, dtype=np.uint8), terms, w, rec["group"], after_keys, after_lo)
+
+    def _phrase_lists(self, phrases: Sequence[Query]) -> int:
+        """Run the positional filter of the batch's phrases on the device (``Engine.phrase_lists``; the same documents
+        as ``FlatIndex.phrase_docs`` minus the deleted ones).  A field's word order is uploaded the first time a phrase
+        on it reaches the engine."""
+        ix, eng = self.ix, self.engine
+        words, slops = [], []
+        for p in phrases:
+            f = ix.field_index(p.fieldname)
+            if f >= 0:
+                if f not in ix.positions:
+                    raise NotImplementedError("field %r was flattened without positions: no phrase queries on it" % p.fieldname)
+                with eng.lock:
+                    if f not in eng.positions_fields:
+                        eng.put_positions(f, *ix.positions[f])
+            tids = [ix.term_id(p.fieldname, w) for w in p.words]
+            words.append([_ffi.TERM_UNKNOWN if t < 0 else t for t in tids])
+            slops.append(min(max(p.slop, 0), 0xFFFFFFFF))          # slop <= 0: no position follows another by <= 0
+        return eng.phrase_lists(words, slops)
 
     # -- searching ----------------------------------------------------------------
     def _run_packed(self, batch: _ffi.PackedBatch, k: int):

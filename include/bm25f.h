@@ -28,9 +28,10 @@
  *          merge + decode + sum of the counts in one call.
  *   bm25f_set_final_date / bm25f_fetch_final / bm25f_merge_final_lists
  *       <- `DateBM25F.final()` of the reference's date-ordered weightings   reference my_whoosh.py:127-154
- *   bm25f_put_lists
+ *   bm25f_put_positions / bm25f_phrase_lists
  *       <- Whoosh's Phrase matcher (quoted phrases of the search form, reference templates/search-form.html:20-40):
- *          the documents that pass the positional test, found on the host, become posting lists of one batch.
+ *          the fields' word order lives in HBM, a positional filter on the device finds the documents that pass,
+ *          and they become posting lists of one batch.  (bm25f_put_lists takes such lists found elsewhere.)
  *   bm25f_submit / bm25f_collect
  *       <- no counterpart in the reference (one request at a time): two batches in flight for servers that batch.
  *   bm25f_get_stats
@@ -278,12 +279,29 @@ int  bm25f_decode_keys(bm25f_handle* h, const uint64_t* d_keys, uint32_t n_queri
  * Whoosh scores a phrase as the AND of its words and lets the positions decide only WHETHER a document matches; the
  * host finds the documents that pass the positional test and hands them over as posting lists with impact 1: list i of
  * this call is leaf_term `*first_term + i` until the next call replaces them all.  A phrase is then the query
- * And(words..., its list) with a tiny positive weight (e.g. 1e-29) on the list's leaf.  Such leaves are served by the
- * warp kernels (k <= 256, <= 32 leaves a query, positive weights, no paging bound); docids are local, strictly
+ * And(words..., its list) with a tiny positive weight (e.g. 1e-29) on the list's leaf.  Such leaves are served by
+ * every kernel (the CTA kernels too: k > 256, more than 32 leaves, paging bounds); docids are local, strictly
  * ascending, < n_docs_all; `offsets` [n_lists + 1] starts at 0.  Waits for the handle's stream; refused while a
  * submitted batch is in flight. */
 #define BM25F_MAX_FILTER_LISTS 4096
 int  bm25f_put_lists(bm25f_handle* h, uint32_t n_lists, const uint64_t* offsets, const uint32_t* docids, uint32_t* first_term);
+
+/* Word order of one field for the positional filter (Whoosh: the positions of a TEXT(phrase=True) field, reference
+ * my_index.py:172-177), document-major as FlatIndex.positions holds it: document d's tokens, as posting-list ids in
+ * document order, are tokens[doc_offsets[d] .. doc_offsets[d + 1]) (doc_offsets [n_docs_all + 1] starts at 0 and never
+ * decreases; a token that is no posting list of the field may be any other value, e.g. 0xFFFFFFFF).  Host pointers,
+ * copied.  A second call for the same field replaces the first; the bytes count in device_bytes.  4 bytes a token. */
+int  bm25f_put_positions(bm25f_handle* h, uint32_t field, const uint64_t* doc_offsets, const uint32_t* tokens);
+/* The positional filter (reference: quoted phrases, search-form.html:20-40; `searcher.search_page(qp, ...)` of a query
+ * that holds them, my_flask.py:208, :211).  Phrase i is words[word_offsets[i] .. word_offsets[i + 1]) (posting-list
+ * ids of one field whose word order was uploaded, at most 32; BM25F_TERM_UNKNOWN makes the list empty) with slops[i]:
+ * a live document matches iff kept_{n-1} is not empty, where kept_0 = the positions of word 0 and kept_j = the
+ * positions p of word j with some e in kept_{j-1}, 1 <= p - e <= slop.  The candidates are the live postings of the
+ * phrase's rarest word.  Afterwards the handle is in the state bm25f_put_lists leaves it in, with phrase i's matches
+ * (ascending) as list i: leaf_term `*first_term + i`.  Same limits (BM25F_MAX_FILTER_LISTS, option filter_postings)
+ * and the same waits and refusals as bm25f_put_lists. */
+int  bm25f_phrase_lists(bm25f_handle* h, uint32_t n_phrases, const uint32_t* word_offsets, const uint32_t* words,
+                        const uint32_t* slops, uint32_t* first_term);
 
 int  bm25f_get_stats(bm25f_handle* h, bm25f_stats* out);
 int  bm25f_reset_stats(bm25f_handle* h);
