@@ -1,9 +1,10 @@
 """Date-ordered weightings (SURVEY.md §8 a10 / f1; reference my_whoosh.py:127-154, selected at
 my_flask.py:183): ``final`` is applied to every match before the top-k (W14).  CPU: the scalar restatement
 against hand-worked values, and the two oracles against each other.  GPU: the device path against the
-oracle.  Final values of documents that share a date differ only in their last few ulps, so parity is an
-absolute tolerance of a few ulps of the final value, and rank by rank the document is the oracle's or one
-that ties with it inside that tolerance."""
+oracle, whose scores are float64 where the engine's are float32: final values of documents that share a date
+differ only in their last few ulps, so parity here is an absolute tolerance of a few ulps of the final value, and
+rank by rank the document is the oracle's or one that ties with it inside that tolerance.  The date orders are
+checked bit for bit, ties inside one final value included, by ``tests/test_gpu_final_exact.py``."""
 from datetime import datetime, timedelta
 
 import numpy as np
