@@ -73,7 +73,7 @@ class Stats(C.Structure):
                 ("tile_docs", C.c_uint32), ("threads", C.c_uint32), ("ctas_per_sm", C.c_uint32),
                 ("packed_payload", C.c_uint32), ("device_bytes", C.c_uint64), ("postings_stream", C.c_uint64),
                 ("postings_team", C.c_uint64), ("postings_cta", C.c_uint64), ("postings_lookup", C.c_uint64),
-                ("reserved0", C.c_uint64), ("ms_stream", C.c_float), ("reserved1", C.c_uint32)]
+                ("postings_topk", C.c_uint64), ("ms_stream", C.c_float), ("reserved1", C.c_uint32)]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}

@@ -404,8 +404,10 @@ __global__ void __launch_bounds__(512) k_score_topk(ScoreParams p) {
   for (uint32_t t = item.tile_begin; t < item.tile_end; ++t) {
     const uint32_t t0 = t * S;
     int* ncand_ctr = &s_ncand[t & 1];
-    // prefetch the boundary row of tile t + 2 (consumed by tile t + 1 as its upper bounds)
-    if (t + 2 <= p.T && tid < L) cp_async4(&s_bounds[(t + 2) % 3][tid], qbounds + (size_t)(t + 2) * L + tid);
+    // prefetch the boundary row of tile t + 2 (consumed by tile t + 1 as its upper bounds).  Every leaf's entry is
+    // loaded whatever the CTA size: a query may have up to MAXL leaves and the CTA as few as 64 threads.
+    if (t + 2 <= p.T)
+      for (int l = tid; l < L; l += nt) cp_async4(&s_bounds[(t + 2) % 3][l], qbounds + (size_t)(t + 2) * L + l);
     const uint32_t* blo = s_bounds[t % 3];
     const uint32_t* bhi = s_bounds[(t + 1) % 3];
 
@@ -2921,6 +2923,7 @@ int bm25f_execute(bm25f_handle* h, bm25f_plan* p) {
   h->stats.postings_stream = p->postings_cls[0];
   h->stats.postings_team = p->postings_cls[1];
   h->stats.postings_cta = p->postings_cls[2];
+  h->stats.postings_topk = p->simple_kernel ? p->postings_cls[2] : 0;
   h->stats.postings_lookup = p->postings_cls[3];
   h->stats.n_items = (uint64_t)p->n_items + p->n_w4 + p->n_w8 + p->n_is;
   h->stats.n_launches = launches;

@@ -174,7 +174,8 @@ typedef struct {
   uint64_t postings_cta;         /* k_score_pipe / k_score_topk */
   uint64_t postings_lookup;      /* k_score_isect: postings of the smallest group are read, the other lists are
                                     searched (skip_to), so most of these postings are NOT read */
-  uint64_t reserved0;
+  uint64_t postings_topk;        /* the part of postings_cta served by k_score_topk rather than k_score_pipe (variant 2,
+                                    or a zero, negative or <= 1e-30 leaf weight anywhere in the batch) */
   float    ms_stream;            /* summed device time of k_score_stream alone (it overlaps k_score_isect) */
   uint32_t reserved1;
 } bm25f_stats;

@@ -237,10 +237,12 @@ def impacts(ix, norm):
 
 
 class Model:
-    """Expected results of packed batches on ``ix`` under ``weighting``."""
+    """Expected results of packed batches on ``ix`` under ``weighting``.  ``fma``: the ``fmaf`` emulation to use
+    (``fma_f32``, or an equal one that is faster on long lists)."""
 
-    def __init__(self, ix, weighting):
+    def __init__(self, ix, weighting, fma=None):
         self.ix = ix
+        self.fma = fma or fma_f32
         self.norm = weighting.norm_tables(ix)
         self.u = impacts(ix, self.norm)
         self.live = np.ones(ix.docids.size, bool) if ix.deleted is None else ix.deleted[ix.docids] == 0
@@ -278,7 +280,7 @@ class Model:
         last = np.full(n, -1, np.int32)
         for i in (plan[::-1] if reverse else plan):
             d, u = self.postings(terms[i])
-            acc[d] = fma_f32(weights[i], u, acc[d])
+            acc[d] = self.fma(weights[i], u, acc[d])
             first = last[d] != groups[i]                    # the document's first leaf of this group (a group's
             cnt[d[first]] += 1                              # leaves are contiguous in the plan)
             last[d] = groups[i]
